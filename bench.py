@@ -2,7 +2,7 @@
 """bench.py — BASELINE.json metric on B200: 512x512 50-step SAM+ControlNet-inpaint images/sec and
 the fused ControlNet x2 + UNet + CFG + DDIM step time.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): SD1.5 topology, 512x512 image -> 64x64 latents, 1 image per
 GPU + classifier-free guidance (B = 2), SAM-ControlNet + inpaint-ControlNet, 77-token context,
@@ -29,6 +29,7 @@ sys.path.insert(0, ROOT)
 STEP_TFLOP = 2.740        # algorithmic 2*MAC per fused step at configs[1] (BASELINE.md §2)
 SAM_TFLOP = 5.96          # SAM ViT-H image encoder, one 1024x1024 image (BASELINE.md §2)
 DDIM_STEPS = 50
+DUMP_MAX_BYTES = 64 << 20
 
 
 def _peaks():
@@ -167,6 +168,17 @@ class GemmProbe:
         return e0.elapsed_time(e1) / reps
 
 
+def dump_outputs(out_dir, **arrays):
+    """Writes each array as out_dir/<name>.npy in float32 so that two builds can be compared output for output; an
+    array over DUMP_MAX_BYTES keeps its leading rows (whole images) up to that size."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        rows = max(1, DUMP_MAX_BYTES // max(1, t[:1].numel() * 4))
+        np.save(os.path.join(out_dir, name + ".npy"), t[:rows].cpu().numpy())
+
+
 def _all_gather_list(t, world):
     import torch.distributed as dist
     bufs = [torch.empty_like(t) for _ in range(world)]
@@ -261,6 +273,8 @@ def run_ours(args, rank, world, local_rank):
     if launches_per_step is None:
         launches_per_step = ops.launch_count() // max(1, args.steps)
     finite = bool(torch.isfinite(eng.latents()).all().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, latents=eng.latents())
 
     # ---- SAM ViT-H encoder (once per image) -----------------------------------------------------
     sam_ms, sam_note, sam = None, "skipped (--no-sam): images/s below is denoise-only", None
@@ -651,7 +665,12 @@ def main():
     ap.add_argument("--images-per-gpu", type=int, default=1,
                     help="images per GPU (network batch = 2x with CFG); 4 = BASELINE.json configs[3]")
     ap.add_argument("--no-batch4", action="store_true", help="skip the extra configs[3] (4 images per GPU) block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what their last step produced (the latents, [images, 4, 64, 64]) "
+                         "as DIR/latents.npy, float32; rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,16 +1,12 @@
 """`EditAnythingLoraModel.process` (SURVEY.md §8b row B1, editanything_b200/app.py):
-  1. against the REFERENCE's own `process` (the method's source compiled out of /root/reference/editany_lora.py,
-     unmodified; the pipelines replaced by spies): both must hand the pipelines the same tensors, PIL images,
-     scales, generator state - i.e. identical pre-processing, control map, inpaint condition, prompt windows, RNG
-     consumption and tile-pass arguments - and return the same structure;
+  1. against the REFERENCE's own `process` (the method's unmodified source, run with the pipelines replaced by
+     spies by oracle/make_golden_ref.py, which records every call in tests/golden/ref_app_process.pt): both must hand
+     the pipelines the same tensors, PIL images, scales, generator state - i.e. identical pre-processing, control
+     map, inpaint condition, prompt windows, RNG consumption and tile-pass arguments - and return the same structure;
   2. end to end on synthetic tiny networks (engines on the CPU emulation of the operators), replaying an
      `input_data.pkl` synthesised the way the reference's decorator writes it (annotator/util.py:75-93)."""
-import ast
 import os
 import pickle
-import random
-import sys
-import textwrap
 from types import SimpleNamespace
 
 import numpy as np
@@ -18,10 +14,9 @@ import pytest
 import torch
 from PIL import Image
 
-from editanything_b200 import app, host
+from editanything_b200 import app
 
-REF = os.environ.get("EA_REFERENCE_ROOT", "/root/reference")
-needs_ref = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "editany_lora.py")), reason="reference tree not present")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 class _Ids(torch.Tensor):
@@ -111,31 +106,36 @@ def _model(cls_or_obj, pipe, tile):
     return m
 
 
-def _reference_class():
-    """The reference's EditAnythingLoraModel with ONLY `process`, `get_sam_control` (their unmodified source) and
-    the module-level helpers they call, compiled in a namespace of stand-ins for the absent third-party imports."""
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import annotator.util as U
-    import cv2
-    import einops
-    src = open(os.path.join(REF, "editany_lora.py")).read()
-    tree = ast.parse(src)
-    ns = {"np": np, "torch": torch, "cv2": cv2, "einops": einops, "random": random, "Image": Image, "PIL": __import__("PIL"),
-          "os": os, "HWC3": U.HWC3, "resize_image": U.resize_image, "get_bounding_box": U.get_bounding_box,
-          "seed_everything": host.seed_everything, "StableDiffusionControlNetInpaintMixingPipeline": type("Mix", (), {}),
-          "prepare_mask_image": None, "obtain_generation_model": None}
-    __import__("PIL.Image")
-    for node in tree.body:
-        if isinstance(node, ast.FunctionDef) and node.name in ("show_anns", "make_inpaint_condition", "get_pipeline_embeds"):
-            exec(compile(ast.Module([node], []), "editany_lora.py", "exec"), ns)
-        if isinstance(node, ast.ClassDef) and node.name == "EditAnythingLoraModel":
-            keep = [n for n in node.body if isinstance(n, ast.FunctionDef) and n.name in ("process", "get_sam_control")]
-            for n in keep:
-                n.decorator_list = []          # @torch.inference_mode() / @save_input_to_file: not part of the arithmetic
-            node.body = keep
-            exec(compile(ast.Module([node], []), "editany_lora.py", "exec"), ns)
-    return ns["EditAnythingLoraModel"]
+def encode(v):
+    """A recorded call / result as plain tensors, lists and dicts (what torch.load reads back without pickle)."""
+    if torch.is_tensor(v):
+        return v.as_subclass(torch.Tensor)       # input_ids and what derives from them are _Ids
+    if isinstance(v, Image.Image):
+        return {"__pil__": v.mode, "__data__": torch.from_numpy(np.array(v))}
+    if isinstance(v, np.ndarray):
+        return {"__ndarray__": torch.from_numpy(v)}
+    if isinstance(v, torch.Generator):
+        return {"__generator__": None}            # compared through the recorded generator_state
+    if isinstance(v, dict):
+        return {k: encode(x) for k, x in v.items()}
+    if isinstance(v, (list, tuple)):
+        return [encode(x) for x in v]
+    return v
+
+
+def decode(v):
+    if isinstance(v, dict) and "__pil__" in v:
+        img = Image.fromarray(v["__data__"].numpy())
+        return img if img.mode == v["__pil__"] else img.convert(v["__pil__"])
+    if isinstance(v, dict) and "__ndarray__" in v:
+        return v["__ndarray__"].numpy()
+    if isinstance(v, dict) and "__generator__" in v:
+        return torch.Generator()
+    if isinstance(v, dict):
+        return {k: decode(x) for k, x in v.items()}
+    if isinstance(v, list):
+        return [decode(x) for x in v]
+    return v
 
 
 def _same(a, b, path=""):
@@ -157,21 +157,17 @@ def _same(a, b, path=""):
         assert a == b, (path, a, b)
 
 
-@needs_ref
 def test_process_hands_the_pipelines_exactly_what_the_reference_does(monkeypatch):
-    monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self)       # the reference hard-codes .cuda()
     monkeypatch.setenv("EA_SAVE_INPUT", "0")
     args, kwargs = _inputs()
-    ref_pipe, ref_tile = SpyPipe(), SpyPipe()
-    ref = _model(_reference_class(), ref_pipe, ref_tile)
-    np.random.seed(5)
-    r_tile, r_res, r_masks, r_prompt = ref.process(*args, **kwargs)
+    ref = decode(torch.load(os.path.join(GOLD, "ref_app_process.pt")))     # the reference's process, np.random.seed(5)
+    r_tile, r_res, r_masks, r_prompt = ref["result"]
     our_pipe, our_tile = SpyPipe(), SpyPipe()
     ours = _model(app.EditAnythingLoraModel, our_pipe, our_tile)
     np.random.seed(5)
     o_tile, o_res, o_masks, o_prompt = ours.process(*args, **kwargs)
-    assert len(ref_pipe.calls) == len(our_pipe.calls) == 1 and len(ref_tile.calls) == len(our_tile.calls) == 2
-    for rc, oc in zip(ref_pipe.calls + ref_tile.calls, our_pipe.calls + our_tile.calls):
+    assert ref["n_main_calls"] == len(our_pipe.calls) == 1 and len(ref["calls"]) - 1 == len(our_tile.calls) == 2
+    for rc, oc in zip(ref["calls"], our_pipe.calls + our_tile.calls):
         # the reference forwards the (unused, None-valued) reference-only keywords as well
         extra = {k: v for k, v in rc.items() if k not in oc}
         assert all(v is None or k.startswith(("attention_auto", "gn_auto", "style_fid", "reference_", "ref_")) for k, v in extra.items()), extra

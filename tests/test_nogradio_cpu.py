@@ -37,7 +37,9 @@ refined, output, ref, text = model.process(*input_data['args'], **input_data['kw
 
 
 @pytest.fixture
-def cpu_backend():
+def cpu_backend(monkeypatch):
+    # the constructors place engines on cuda:0 whenever a GPU is present; the emulated operators work on CPU tensors
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
     _backend.OPS = cpu_ops
     yield
     _backend.OPS = None

@@ -1,5 +1,5 @@
 """CPU suite for the first-stage decoder (SURVEY.md §8f N1): the oracle restatement against the
-reference's own `Decoder` (imported from /root/reference when present) and against the
+outputs of the reference's own `Decoder` / `Encoder` (recorded by oracle/make_golden_ref.py) and against the
 reference-generated golden vectors; the host-side graph of editanything_b200.vae with the operators
 emulated on CPU (tests/cpu_ops.py); the diffusers -> ldm key map."""
 import os
@@ -11,7 +11,6 @@ from editanything_b200.vae import DiagonalGaussian, VaeDecoderEngine, VaeEncoder
 from editanything_b200.vae_spec import (SD_VAE, VAE_TINY, make_vae_state_dict, vae_decoder_param_shapes,
                                         vae_encoder_param_shapes)
 from editanything_b200.weights import vae_diffusers_to_ldm, vae_ldm_to_diffusers_names
-from oracle import ref_shim
 from oracle import vae_oracle as V
 from oracle.make_golden_vae import make_image, make_latents
 from tests import cpu_ops
@@ -29,15 +28,14 @@ def test_param_count_matches_kl_f8_decoder():
     assert abs(n - 49.49e6) < 0.05e6, n      # SURVEY.md §8a R17: 49.5 M parameters
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_oracle_matches_reference_decoder():
     cfg = VAE_TINY
     sd = make_vae_state_dict(cfg, 21)
     z = make_latents(cfg, 2, 12, 5) / cfg.scaling_factor
-    ref = V.reference_decoder(cfg, sd)(z)
+    ref = torch.load(os.path.join(GOLD, "ref_vae_modules.pt"))["decoded"]      # the reference's Decoder(z)
     with torch.no_grad():
         ours = V.decode(z, sd, cfg)
-    assert (ours - ref).abs().max().item() < 2e-5
+    assert ours.shape == ref.shape and (ours - ref).abs().max().item() < 2e-5
 
 
 def test_oracle_reproduces_reference_golden():
@@ -96,12 +94,11 @@ def test_param_count_matches_kl_f8_encoder():
     assert abs(n - 34.16e6) < 0.05e6, n      # SURVEY.md §8a R6: 34.2 M parameters
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_encode_oracle_matches_reference_encoder():
     cfg = VAE_TINY
     sd = make_vae_state_dict(cfg, 31, part="encoder")
     x = make_image(2, 24, 6)              # odd spatial size after the stride-2: exercises the (0,1,0,1) padding
-    ref = V.reference_encoder(cfg, sd)(x)
+    ref = torch.load(os.path.join(GOLD, "ref_vae_modules.pt"))["moments"]      # the reference's Encoder(x)
     with torch.no_grad():
         ours = V.encode_moments(x, sd, cfg)
     assert ours.shape == ref.shape and (ours - ref).abs().max().item() < 2e-5
